@@ -2,7 +2,7 @@
 configuration the headline metric `audio-sec/sec` is quoted on; it fits one B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--duration 30] [--batch 8]
-                  [--scaling weak|strong] [--scale small|medium|large] [--workload musicgen|encodec]
+                  [--scaling weak|strong] [--scale small|medium|large] [--workload musicgen|encodec] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...
 
 Defaults = BASELINE configs[2] with `--batch` items PER GPU (`scaling: weak`, as the contract prescribes for a path that shards
@@ -16,6 +16,10 @@ by EnCodec decode of the tokens to audio.  `value` = audio seconds produced by a
 inputs (condition tensors) resident in HBM.  `e2e` = the same through the public MusicGen.generate(descriptions) call
 with host inputs (text-encoder states pinned on the host, copied inside the timed region) and the waveform read back.
 Weights are seeded random (no checkpoints offline), inputs synthetic.
+
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 as DIR/<name>.npy (float32): `tokens` [B, K, T] and
+`wav` [B, 1, samples] for MusicGen, `codes` and `wav` for EnCodec (see dump_outputs for outputs over 64 MB).  Inputs, weights
+and sampling seeds are fixed, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the reference's OWN code on the box's host cores: the unmodified package installed under
 baseline/_ref (baseline/install_ref.sh; it ships with the snapshot), driven through oracle/ref_import.py's third-party
@@ -113,6 +117,26 @@ def dist_setup(n):
     return rank, world
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict):
+    """Write each tensor of `arrays` as `path`/<name>.npy in float32.  When together they exceed DUMP_LIMIT_BYTES, every
+    array is flattened and keeps the same fraction of its elements, at sorted positions drawn from a fixed seed: the sample
+    is the same in every run, so two dumps still compare element for element."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().to('cpu', torch.float32) for k, v in arrays.items()}
+    total = sum(v.numel() for v in arrays.values())
+    budget = (DUMP_LIMIT_BYTES - 1024 * len(arrays)) // 4       # float32 elements; 1 KB per file for the .npy header
+    for name, v in arrays.items():
+        if total > budget:
+            n = v.numel() * budget // total
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(path, f'{name}.npy'), v.numpy())
+
+
 def encodec_roofline(samples: int, ms: float):
     """SURVEY.md section 8d for EnCodec-32k encode+decode: 4 822 B/sample when every layer reads its input and writes its
     output once (fp32, ELU / residual / padding fused) and 486 kFLOP/sample.  With tensor-core convolutions the per-layer design
@@ -154,7 +178,7 @@ def run_encodec(args):
         outs = []
         for i in range(0, B, CH):
             codes, scale = cm.encode(x_dev[i:i + CH])
-            outs.append(cm.decode(codes, scale))
+            outs.append((codes, cm.decode(codes, scale)))
         return outs
 
     def step_e2e():
@@ -190,12 +214,16 @@ def run_encodec(args):
         return ms, out
 
     for _ in range(args.warmup):
-        l0 = cm.launches
         step_device()
-        launches = cm.launches - l0
+    l0 = cm.launches
     with ClockSampler(torch.cuda.current_device()) as clk:
-        ms, _ = timed(step_device, args.steps)
+        ms, outs = timed(step_device, args.steps)
     clocks = clk.summary()
+    launches = (cm.launches - l0) // args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(codes=torch.cat([c.cpu() for c, _ in outs]),
+                                             wav=torch.cat([w.cpu() for _, w in outs])))
+    del outs
     ms_e2e, _ = timed(step_e2e, max(1, min(args.steps, 3)))
     n_e2e = max(1, min(args.steps, 3))
     samples_step = total_items * n_samp
@@ -283,7 +311,7 @@ def run_b200(args):
         if strong and world > 1:   # configs[2] read literally: one batch over the ranks, the audio gathered on every rank
             from audiocraft_b200.dist import gather_batch
             wav = gather_batch(wav, args.batch)
-        return wav
+        return tokens, wav
 
     def step_e2e():
         cond_mod.encoder = pinned_encoder
@@ -318,13 +346,16 @@ def run_b200(args):
         return ms, out
 
     for _ in range(args.warmup):
-        l0 = cm.launches
-        wav = step_device()
-        dec_launches = cm.launches - l0   # EnCodec decode kernels per generate
+        step_device()
     torch.cuda.synchronize()
+    l0 = cm.launches
     with ClockSampler(torch.cuda.current_device()) as clk:
-        ms, wav = timed(step_device, args.steps)
+        ms, (tokens, wav) = timed(step_device, args.steps)
     clocks = clk.summary()
+    dec_launches = (cm.launches - l0) // args.steps   # EnCodec decode kernels per generate
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(tokens=tokens, wav=wav))
+    del tokens, wav
     audio_s = total_items * dur * args.steps
     value = audio_s / (ms / 1e3)
     n_e2e = max(1, min(args.steps, 3))
@@ -544,7 +575,12 @@ if __name__ == '__main__':
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-ref-gpu', action='store_true', help='skip timing the reference CUDA path (reference_gpu block)')
     ap.add_argument('--no-encodec', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs applies to --impl b200')
     if a.impl == 'reference':
         run_reference(a)
     elif a.workload == 'encodec':

@@ -184,6 +184,48 @@ def golden_lm_fullsize(name, batch, t_text=16, T=1500, wseed=0, cseed=3, sseed=1
     print(name, 'fullsize logits', tuple(tv.shape), f'{time.time() - t0:.0f} s')
 
 
+def golden_lm_fullsize_cuda(name, batch, items, t_text=16, T=1500, wseed=0, cseed=3, sseed=17, n_top=8, n_cols=56):
+    """The reference's own CUDA path at the benchmarked shapes (needs a GPU): fp16 transformer under autocast, SDPA
+    (audiocraft/models/loaders.py:115-118, genmodel.py:74-78), one causal forward over a seeded delay-pattern sequence of
+    T frames with the CFG rows [cond; null] = 2*batch, weights generated on CUDA in fp16 exactly as the test regenerates
+    them.  The full per-row logits ([7, 2*batch, K, card]) are too large to store, so the fixture keeps, for the batch
+    items `items` (both CFG rows of each), the top-`n_top` logits of every row plus the logits at `n_cols` seeded columns,
+    and for EVERY item the argmax and top-2 margin of the CFG-mixed logits.  The logits are fp16 values under autocast and
+    are stored as such (lossless)."""
+    import time
+    t0 = time.time()
+    dev = torch.device('cuda')
+    cfg = synth.lm_config(name)
+    sd = synth.synth_lm_state_dict(cfg, seed=wseed, device='cuda', dtype=torch.float16)
+    w_head = sd['emb.0.weight'][:2, :16].cpu().clone()
+    hid, mask = synth.synth_text_condition(cfg, batch, t_text, seed=cseed)
+    from oracle import ref_models as RM
+    ref, CA = RM.build_ref_lm(cfg, sd, RM.text_table(hid, mask, cfg['cond_dim']), device=dev, dtype=torch.float16)
+    del sd
+    seq = H.fullsize_sequence(cfg, batch, T, sseed).to(dev)
+    S = seq.shape[-1]
+    cc = RM.ref_cfg_conditions(ref, CA, batch)                           # {'description': ([2B,T,d] fp32, mask)}
+    with torch.autocast('cuda', dtype=torch.float16):
+        rl = ref(torch.cat([seq, seq], 0)[..., :S - 1], conditions=[], condition_tensors=cc)   # [2B,K,S-1,card]
+    rl = rl[:, :, FULLSIZE_STEPS, :].float().permute(2, 0, 1, 3).contiguous().cpu()          # [n,2B,K,card]
+    c, u = rl.split(batch, dim=1)
+    rmix = u + (c - u) * cfg['cfg_coef']
+    top2 = rmix.topk(2, dim=-1)
+    rows = torch.tensor(list(items) + [batch + i for i in items])
+    sub = rl[:, rows]
+    tv, ti = sub.topk(n_top, dim=-1)
+    g = torch.Generator()
+    g.manual_seed(1000 + batch)
+    cols = torch.randperm(cfg['card'], generator=g)[:n_cols].sort().values
+    out = dict(name=name, batch=batch, t_text=t_text, T=T, wseed=wseed, cseed=cseed, sseed=sseed, steps=FULLSIZE_STEPS,
+               w_head=w_head, cross_rowsum=cc['description'][0].float().sum(-1).cpu(), rows=rows,
+               top_v=tv.half(), top_i=ti.to(torch.int16), cols=cols.to(torch.int16), cols_v=sub[..., cols].half(),
+               mix_argmax=top2.indices[..., 0].to(torch.int16), mix_margin=top2.values[..., 0] - top2.values[..., 1])
+    assert torch.equal(out['top_v'].float(), tv) and torch.equal(out['cols_v'].float(), sub[..., cols])
+    torch.save(out, os.path.join(H.GOLDEN_DIR, f'{name}_cuda_autocast.pt'))
+    print(name, 'reference CUDA autocast logits', tuple(rl.shape), 'kept rows', rows.tolist(), f'{time.time() - t0:.0f} s')
+
+
 def golden_encodec_fullsize():
     """BASELINE config 1 at its real length (10 s = 240 000 samples at 24 kHz: codes [1, n_q, 750] for n_q = 8 and 32)
     and a [2, 1, 320000] slice of config 4 (32 kHz, 4 codebooks): codes from the reference (int16 to keep the fixture small)."""
@@ -273,6 +315,10 @@ if __name__ == '__main__':
         golden_encodec_fullsize()
         golden_lm_fullsize('musicgen_medium', 8)
         golden_lm_fullsize('musicgen_large', 4)
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == 'fullsize_cuda':   # on a CUDA device
+        golden_lm_fullsize_cuda('musicgen_medium', 8, items=range(8))
+        golden_lm_fullsize_cuda('musicgen_large', 32, items=[0, 5, 10, 15, 16, 21, 26, 31])
         sys.exit(0)
     golden_patterns()
     golden_sampling()

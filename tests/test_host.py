@@ -64,8 +64,9 @@ def test_fused_residual_block_routing():
 
 def test_sass_is_sm100a():
     import subprocess
-    from audiocraft_b200 import _lib
-    out = subprocess.run(['cuobjdump', '-lelf', _lib.LIB_PATH], capture_output=True, text=True).stdout
+    from audiocraft_b200 import _lib, build
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), 'cuobjdump')   # the toolkit that built the library, on PATH or not
+    out = subprocess.run([cuobjdump, '-lelf', _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert 'sm_100a' in out, out
 
 
