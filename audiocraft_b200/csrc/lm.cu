@@ -39,7 +39,8 @@ __device__ __forceinline__ void mma16816(float (&c)[4], uint32_t a0, uint32_t a1
 
 // Programmatic dependent launch (PDL): a kernel launched with the programmatic-stream-serialization attribute may
 // start while its predecessor is still running; everything before pdl_wait() must only touch memory no earlier
-// kernel of the step writes (weights).  Both are no-ops for a normally launched kernel.
+// kernel of the step writes (weights, LayerNorm parameters, the cross K/V, cache positions < pos: see
+// enqueue_step_kernels).  Both are no-ops for a normally launched kernel.
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
@@ -204,11 +205,14 @@ struct GemmParams {
 // CTA = 4 warps, tile = 16 output features x kslice of K.  The CTA's 16 x kslice weight slab is fetched by ONE thread
 // with 16 TMA bulk copies (one per W row, padded pitch => conflict-free fragment reads) BEFORE griddepcontrol.wait, i.e.
 // while the producer of the activations is still running: under PDL the weight stream of kernel n+1 overlaps kernel n.
-// FT2 = feature tiles of 16 per CTA.  FT2 = 2 (opt-in per GEMM, see pick_ft2) halves the number of CTAs and therefore
-// the activation traffic out of L2: every CTA re-reads the whole 16 x K activation block, and the in-kernel timeline
-// (profiles/r1_lm_timeline_layer0_kv1_fine.log) shows the k-loop of the big GEMMs bound by exactly that (14 MB of
-// activation reads per 14 MB weight matrix; ~0.8 us per dependent batch of loads).
-template <int NT, int EPI, int FT2 = 1>
+// FT2 = feature tiles of 16 per CTA (1, 2 or 3; see pick_tiling).  Wider tiles mean fewer CTAs and therefore less
+// activation traffic out of L2: every CTA reads the whole (8*NT) x kslice activation block.
+// STAGED: right after griddepcontrol.wait, warp 0 copies that activation block into shared memory with one TMA bulk copy
+// per row (same padded pitch as the weight slab), so the k-loop waits for ONE round trip and then reads only shared
+// memory.  Without it (register loads) every warp fetches its activation fragments in dependent batches of U k-blocks:
+// at 12 k-blocks per warp that was 3 batches, ~0.8 us each (profiles/r1_lm_timeline_layer0_kv1_fine.log).  Both paths
+// issue the same MMAs in the same order, so their results are bit-identical.
+template <int NT, int EPI, int FT2 = 1, bool STAGED = false>
 __global__ void __launch_bounds__(128) lm_gemm_kernel(GemmParams p) {
 #ifndef ACB_GEMM_U2
 #define ACB_GEMM_U2 4   // k-blocks per batch of activation loads at <= 16 rows (experiment builds: -DACB_GEMM_U2=6)
@@ -221,12 +225,16 @@ __global__ void __launch_bounds__(128) lm_gemm_kernel(GemmParams p) {
     const int f0 = blockIdx.x * FB;
     const int k0 = blockIdx.y * p.kslice;
     const int ks = min(p.kslice, p.K - k0);          // elements of K this CTA reduces over
-    const int pitch = p.kslice * 2 + 64;             // bytes per staged W row (+64: conflict-free LDS.128)
-    uint64_t* bar = reinterpret_cast<uint64_t*>(gsm + FB * pitch);
-    float* red = reinterpret_cast<float*>(gsm + FB * pitch + 16);   // [4][FB][RP]
+    const int pitch = p.kslice * 2 + 64;             // bytes per staged W / X row (+64: conflict-free LDS.128)
+    unsigned char* xs = gsm + FB * pitch;            // STAGED: [8*NT][pitch] activation block
+    uint64_t* bar = reinterpret_cast<uint64_t*>(xs + (STAGED ? 8 * NT * pitch : 0));   // [0] weights, [1] activations
+    float* red = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(bar) + 16);   // [4][FB][RP]
 
     tl_stamp(p.timing, 0);
-    if (tid == 0) mbar_init(bar, 1);
+    if (tid == 0) {
+        mbar_init(bar, 1);
+        if (STAGED) mbar_init(bar + 1, 1);
+    }
     __syncthreads();
     if (tid == 0) {
         mbar_expect_tx(bar, (uint32_t)FB * (uint32_t)ks * 2u);
@@ -237,6 +245,13 @@ __global__ void __launch_bounds__(128) lm_gemm_kernel(GemmParams p) {
     pdl_trigger();
     pdl_wait();   // activations written by the previous kernel are visible from here on
     tl_stamp(p.timing, 1);
+    if (STAGED && warp == 0) {
+        if (lane == 0) mbar_expect_tx(bar + 1, 8u * NT * (uint32_t)ks * 2u);
+        __syncwarp();
+#pragma unroll 1
+        for (int r = lane; r < 8 * NT; r += 32)
+            bulk_g2s(xs + r * pitch, p.X + (size_t)r * p.K + k0, (uint32_t)ks * 2u, bar + 1);
+    }
     int cache_pos = 0;
     if (EPI == EPI_QKV || EPI == EPI_QKV_PF) cache_pos = p.pos[0];   // requested now, consumed in the epilogue: off the critical path
 
@@ -254,7 +269,31 @@ __global__ void __launch_bounds__(128) lm_gemm_kernel(GemmParams p) {
     const unsigned char* wr1 = wr0 + 8 * pitch;
 
     bool w_ready = false;
-    for (int kb = kb0; kb < kb1; kb += U) {
+    if (STAGED) {
+        mbar_wait(bar, 0);
+        tl_stamp(p.timing, 4);
+        mbar_wait(bar + 1, 0);
+        tl_stamp(p.timing, 7);
+        w_ready = true;
+        const unsigned char* xg = xs + g * pitch + 16 * c4;
+#pragma unroll 2
+        for (int kb = kb0; kb < kb1; ++kb) {
+            uint4 xv[NT];
+#pragma unroll
+            for (int j = 0; j < NT; ++j) xv[j] = *reinterpret_cast<const uint4*>(xg + 8 * j * pitch + kb * 64);
+#pragma unroll
+            for (int ft = 0; ft < FT2; ++ft) {
+                const uint4 wa = *reinterpret_cast<const uint4*>(wr0 + ft * 16 * pitch + kb * 64);
+                const uint4 wb = *reinterpret_cast<const uint4*>(wr1 + ft * 16 * pitch + kb * 64);
+#pragma unroll
+                for (int j = 0; j < NT; ++j) {
+                    mma16816(c[ft][j], wa.x, wb.x, wa.y, wb.y, xv[j].x, xv[j].y);
+                    mma16816(c[ft][j], wa.z, wb.z, wa.w, wb.w, xv[j].z, xv[j].w);
+                }
+            }
+        }
+    }
+    for (int kb = kb0; !STAGED && kb < kb1; kb += U) {
         uint4 xv[U][NT];
 #pragma unroll
         for (int u = 0; u < U; ++u)
@@ -531,8 +570,9 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) lm_attn2_kernel(AttnParams p) 
     const int sl = lane & 7, pg = lane >> 3;
     tl_stamp(p.timing, 0);
     pdl_trigger();
-    pdl_wait();
-    tl_stamp(p.timing, 1);
+    // Before griddepcontrol.wait: pos and every cache position < pos are final for the whole step (see enqueue_step_kernels: the
+    // step's first kernel waits for everything enqueued before it), so the first ATT2_DEPTH - 1 ring stages are filled while the
+    // QKV GEMM still runs.  Position pos itself is what that GEMM writes: it is skipped here and fetched after the wait.
     const int n = p.fixed_len > 0 ? p.fixed_len : p.pos[0] + 1;
     const size_t base = ((size_t)row * p.H + h) * p.cache_len * 64 + sl * 8;
     const __half* kb = p.kc + base;
@@ -540,10 +580,10 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) lm_attn2_kernel(AttnParams p) 
     const uint32_t ring = smem_u32(att2sm) + (uint32_t)(warp * ATT2_DEPTH * 1024 + lane * 16);
     // iteration k of this warp covers positions (k * 8 + warp) * 4 + pg
     const int n_it = (n + 31 - warp * 4) / 32 > 0 ? (n - warp * 4 + 31) / 32 : 0;   // iterations with at least one live position group
-    auto issue = [&](int k) {
+    auto issue = [&](int k, int lim) {   // copies of positions < lim; every lane commits one group per call, empty or not
         if (k < n_it) {
             const int pp = (k * ATT_WARPS + warp) * 4 + pg;
-            if (pp < n) {
+            if (pp < lim) {
                 const uint32_t d = ring + (uint32_t)((k % ATT2_DEPTH) * 1024);
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(kb + (size_t)pp * 64) : "memory");
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d + 512u), "l"(vb + (size_t)pp * 64) : "memory");
@@ -552,7 +592,18 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) lm_attn2_kernel(AttnParams p) 
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
 #pragma unroll
-    for (int k = 0; k < ATT2_DEPTH - 1; ++k) issue(k);
+    for (int k = 0; k < ATT2_DEPTH - 1; ++k) issue(k, n - 1);
+    pdl_wait();
+    tl_stamp(p.timing, 1);
+    // Position n - 1: if it fell into the stages above, its 8 lanes load it now (together with q) and put it into the slot of its
+    // iteration, which no copy targets until this lane's loop has read it (same thread: no barrier needed).
+    const int pl = n - 1, kl = pl >> 5;
+    const bool own_last = kl < ATT2_DEPTH - 1 && ((pl >> 2) & (ATT_WARPS - 1)) == warp && (pl & 3) == pg;
+    uint4 lk = make_uint4(0, 0, 0, 0), lv = lk;
+    if (own_last) {
+        lk = *reinterpret_cast<const uint4*>(kb + (size_t)pl * 64);
+        lv = *reinterpret_cast<const uint4*>(vb + (size_t)pl * 64);
+    }
 
     float q[8];
     {
@@ -562,6 +613,11 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) lm_attn2_kernel(AttnParams p) 
         q[3] = half_round(qa.w) * p.scale; q[4] = half_round(qb.x) * p.scale; q[5] = half_round(qb.y) * p.scale;
         q[6] = half_round(qb.z) * p.scale; q[7] = half_round(qb.w) * p.scale;
     }
+    if (own_last) {
+        const uint32_t d = ring + (uint32_t)(kl * 1024);
+        asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(d), "r"(lk.x), "r"(lk.y), "r"(lk.z), "r"(lk.w) : "memory");
+        asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(d + 512u), "r"(lv.x), "r"(lv.y), "r"(lv.z), "r"(lv.w) : "memory");
+    }
     tl_stamp(p.timing, 4);
     OnlineSM st;
     st.m = -INFINITY; st.l = 0.f;
@@ -569,7 +625,7 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) lm_attn2_kernel(AttnParams p) 
     for (int e = 0; e < 8; ++e) st.acc[e] = 0.f;
 
     for (int k = 0; k < n_it; ++k) {                 // warp-uniform trip count (the shuffles need all 32 lanes)
-        issue(k + ATT2_DEPTH - 1);
+        issue(k + ATT2_DEPTH - 1, n);
         asm volatile("cp.async.wait_group %0;" ::"n"(ATT2_DEPTH - 1) : "memory");   // iteration k's copies of this lane have landed
         const int pp = (k * ATT_WARPS + warp) * 4 + pg;
         const uint32_t sa = ring + (uint32_t)((k % ATT2_DEPTH) * 1024);
@@ -638,18 +694,36 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) lm_attn2_kernel(AttnParams p) 
 }
 
 // Cross attention over the (short) text condition: one WARP per (row, head), lane = text position for the scores,
-// lane = 2 output dims for the weighted sum.  K/V were computed once per generate() (acb_lm_begin).
+// lane = 2 output dims for the weighted sum.  K/V were computed once per generate() (acb_lm_begin) and no kernel of a step
+// writes them (see enqueue_step_kernels: the step's first kernel waits for everything enqueued before it), so the first
+// chunk of 32 text positions -- K row per lane, V pair of dims per lane -- is loaded into registers BEFORE
+// griddepcontrol.wait; after it only the query partials are read.  Later chunks are loaded after the wait.
 template <bool PF>
 __global__ void __launch_bounds__(256) lm_cross_attn_kernel(AttnParams p, int rows) {
     __shared__ float qs[8][64];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int pair = blockIdx.x * 8 + warp;          // (row, head) index
+    const bool live = pair < rows * p.H;             // warp-uniform
+    const int row = pair / p.H, h = pair % p.H, n = p.fixed_len;
+    const size_t base = ((size_t)(PF ? row % p.rows_real : row) * p.H + h) * p.cache_len * 64;   // K / V of the generation row
+    uint4 kr[8];                                     // K of text position t0 + lane
+    __half2 vr[32];                                  // V[t0 + j][2 lane .. 2 lane + 1]
+    auto load_chunk = [&](int t0) {
+        const int t = t0 + lane;
+#pragma unroll
+        for (int c = 0; c < 8; ++c)
+            kr[c] = t < n ? reinterpret_cast<const uint4*>(p.kc + base + (size_t)t * 64)[c] : make_uint4(0, 0, 0, 0);
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+            vr[j] = t0 + j < n ? *reinterpret_cast<const __half2*>(p.vc + base + (size_t)(t0 + j) * 64 + lane * 2)
+                               : __floats2half2_rn(0.f, 0.f);
+    };
     tl_stamp(p.timing, 0);
+    if (live) load_chunk(0);
     pdl_trigger();
     pdl_wait();
     tl_stamp(p.timing, 1);
-    if (pair >= rows * p.H) return;                  // warp-uniform
-    const int row = pair / p.H, h = pair % p.H, n = p.fixed_len;
+    if (!live) return;
     {
         const float* qp = p.q + (size_t)row * p.d + h * 64 + lane * 2;
         float2 part[ACB_LM_MAX_SPLIT];
@@ -664,18 +738,16 @@ __global__ void __launch_bounds__(256) lm_cross_attn_kernel(AttnParams p, int ro
     }
     __syncwarp();
     tl_stamp(p.timing, 4);
-    const size_t base = ((size_t)(PF ? row % p.rows_real : row) * p.H + h) * p.cache_len * 64;   // K / V of the generation row
     float mx = -INFINITY, l = 0.f, o0 = 0.f, o1 = 0.f;
     for (int t0 = 0; t0 < n; t0 += 32) {             // chunks of 32 text positions (online softmax across chunks)
+        if (t0 > 0) load_chunk(t0);
         const int t = t0 + lane;
         float s = -INFINITY;
         if (t < n) {
-            const uint4* kr = reinterpret_cast<const uint4*>(p.kc + base + (size_t)t * 64);
             s = 0.f;
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
-                const uint4 kk = kr[c];
-                const __half2* k2 = reinterpret_cast<const __half2*>(&kk);
+                const __half2* k2 = reinterpret_cast<const __half2*>(&kr[c]);
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
                     const float2 f = __half22float2(k2[e]);
@@ -691,12 +763,14 @@ __global__ void __launch_bounds__(256) lm_cross_attn_kernel(AttnParams p, int ro
         l = l * corr + warp_sum(pw);
         o0 *= corr; o1 *= corr;
         tl_stamp(p.timing, 6);
-        const int cnt = min(32, n - t0);
-        for (int j = 0; j < cnt; ++j) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
             const float wj = __shfl_sync(0xffffffffu, pw, j);
-            const float2 f = __half22float2(*reinterpret_cast<const __half2*>(p.vc + base + (size_t)(t0 + j) * 64 + lane * 2));
-            o0 = fmaf(wj, f.x, o0);
-            o1 = fmaf(wj, f.y, o1);
+            if (t0 + j < n) {
+                const float2 f = __half22float2(vr[j]);
+                o0 = fmaf(wj, f.x, o0);
+                o1 = fmaf(wj, f.y, o1);
+            }
         }
         mx = cm;
     }
@@ -921,7 +995,7 @@ struct acb_lm {
     cudaStream_t capture_stream = nullptr;
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t exec = nullptr;
-    int batch = 0, rows = 0, rows_pad = 0, text_len = 0, seq_len = 0, sms = 148;
+    int batch = 0, rows = 0, rows_pad = 0, text_len = 0, seq_len = 0, sms = 148, smem_per_sm = 228 * 1024;
     int launches = 0;
     bool has_cross = false;
     bool pdl = true;          // programmatic dependent launch between the kernels of a step
@@ -956,64 +1030,102 @@ static cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
 
 static int nt_for_rows(int rows) { return rows <= 8 ? 1 : (rows <= 16 ? 2 : (rows <= 32 ? 4 : 8)); }
 
-static size_t gemm_smem_bytes(int nt, int kslice, int ft2 = 1) {
-    return (size_t)16 * ft2 * (kslice * 2 + 64) + 16 + (size_t)4 * 16 * ft2 * (8 * nt + 1) * sizeof(float);
+static size_t gemm_smem_bytes(int nt, int kslice, int ft2, bool staged) {
+    const size_t pitch = (size_t)kslice * 2 + 64;
+    return 16 * ft2 * pitch + (staged ? 8 * nt * pitch : 0) + 16 + (size_t)4 * 16 * ft2 * (8 * nt + 1) * sizeof(float);
 }
-constexpr int GEMM_MAX_SMEM = 120 * 1024;
+// Register-load tiles stay within 120 KB so that two CTAs share an SM; staged tiles may use all an SM allows one block.
+constexpr int GEMM_REG_MAX_SMEM = 120 * 1024, GEMM_MAX_SMEM = 227 * 1024;
 
-template <int EPI, int FT2>
+struct GemmTiling { int ft2; bool staged; };
+
+template <int EPI, int FT2, bool STAGED>
 static int launch_gemm_ft(int nt, const GemmParams& p, int nsplit, cudaStream_t s, bool pdl) {
     dim3 grid(p.N / (16 * FT2), nsplit);
-    const size_t smem = gemm_smem_bytes(nt, p.kslice, FT2);
-    ACB_REQUIRE(smem <= (size_t)GEMM_MAX_SMEM && p.N % (16 * FT2) == 0, "lm_gemm: tile does not fit (N=%d kslice=%d ft2=%d)", p.N, p.kslice, FT2);
+    const size_t smem = gemm_smem_bytes(nt, p.kslice, FT2, STAGED);
+    ACB_REQUIRE(smem <= (size_t)GEMM_MAX_SMEM && p.N % (16 * FT2) == 0, "lm_gemm: tile does not fit (N=%d kslice=%d ft2=%d staged=%d)",
+                p.N, p.kslice, FT2, (int)STAGED);
     switch (nt) {
-        case 1: ACB_LAUNCH((lm_gemm_kernel<1, EPI, FT2>), grid, dim3(128), smem, s, pdl, p); break;
-        case 2: ACB_LAUNCH((lm_gemm_kernel<2, EPI, FT2>), grid, dim3(128), smem, s, pdl, p); break;
-        case 4: ACB_LAUNCH((lm_gemm_kernel<4, EPI, FT2>), grid, dim3(128), smem, s, pdl, p); break;
-        default: ACB_LAUNCH((lm_gemm_kernel<8, EPI, FT2>), grid, dim3(128), smem, s, pdl, p); break;
+        case 1: ACB_LAUNCH((lm_gemm_kernel<1, EPI, FT2, STAGED>), grid, dim3(128), smem, s, pdl, p); break;
+        case 2: ACB_LAUNCH((lm_gemm_kernel<2, EPI, FT2, STAGED>), grid, dim3(128), smem, s, pdl, p); break;
+        case 4: ACB_LAUNCH((lm_gemm_kernel<4, EPI, FT2, STAGED>), grid, dim3(128), smem, s, pdl, p); break;
+        default: ACB_LAUNCH((lm_gemm_kernel<8, EPI, FT2, STAGED>), grid, dim3(128), smem, s, pdl, p); break;
     }
     return ACB_OK;
 }
+// The cross K/V and prefill QKV epilogues are built with 16-feature register-load tiles only.
+constexpr bool gemm_epi_tiled(int epi) { return epi != EPI_CROSSKV && epi != EPI_QKV_PF; }
+
 template <int EPI>
-static int launch_gemm(int nt, const GemmParams& p, int nsplit, cudaStream_t s, bool pdl, int ft2 = 1) {
-    if (ft2 == 2) {
-        if constexpr (EPI == EPI_CROSSKV || EPI == EPI_QKV_PF) { acb_set_error("lm_gemm: this epilogue uses 16-feature tiles"); return ACB_ERR_INVALID; }
-        else return launch_gemm_ft<EPI, 2>(nt, p, nsplit, s, pdl);
+static int launch_gemm(int nt, const GemmParams& p, int nsplit, cudaStream_t s, bool pdl, GemmTiling t = {1, false}) {
+    if constexpr (gemm_epi_tiled(EPI)) {
+        if (t.staged) {
+            if (t.ft2 == 3) return launch_gemm_ft<EPI, 3, true>(nt, p, nsplit, s, pdl);
+            if (t.ft2 == 2) return launch_gemm_ft<EPI, 2, true>(nt, p, nsplit, s, pdl);
+            return launch_gemm_ft<EPI, 1, true>(nt, p, nsplit, s, pdl);
+        }
+        if (t.ft2 == 2) return launch_gemm_ft<EPI, 2, false>(nt, p, nsplit, s, pdl);
+    } else if (t.staged || t.ft2 != 1) {
+        acb_set_error("lm_gemm: this epilogue uses 16-feature register-load tiles");
+        return ACB_ERR_INVALID;
     }
-    return launch_gemm_ft<EPI, 1>(nt, p, nsplit, s, pdl);
+    return launch_gemm_ft<EPI, 1, false>(nt, p, nsplit, s, pdl);
 }
 
-template <int NT, int EPI, int FT2>
+template <int NT, int EPI, int FT2, bool STAGED>
 static cudaError_t gemm_attr_one() {
-    cudaError_t e = cudaFuncSetAttribute(lm_gemm_kernel<NT, EPI, FT2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_MAX_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(lm_gemm_kernel<NT, EPI, FT2, STAGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_MAX_SMEM);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(lm_gemm_kernel<NT, EPI, FT2>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    return cudaFuncSetAttribute(lm_gemm_kernel<NT, EPI, FT2, STAGED>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+}
+template <int EPI, int FT2, bool STAGED>
+static cudaError_t gemm_attr_nt() {
+    cudaError_t e;
+    if ((e = gemm_attr_one<1, EPI, FT2, STAGED>()) != cudaSuccess) return e;
+    if ((e = gemm_attr_one<2, EPI, FT2, STAGED>()) != cudaSuccess) return e;
+    if ((e = gemm_attr_one<4, EPI, FT2, STAGED>()) != cudaSuccess) return e;
+    return gemm_attr_one<8, EPI, FT2, STAGED>();
 }
 template <int EPI>
 static cudaError_t gemm_attr_all() {
     cudaError_t e;
-    if ((e = gemm_attr_one<1, EPI, 1>()) != cudaSuccess) return e;
-    if ((e = gemm_attr_one<2, EPI, 1>()) != cudaSuccess) return e;
-    if ((e = gemm_attr_one<4, EPI, 1>()) != cudaSuccess) return e;
-    if ((e = gemm_attr_one<8, EPI, 1>()) != cudaSuccess) return e;
-    if constexpr (EPI != EPI_CROSSKV && EPI != EPI_QKV_PF) {
-        if ((e = gemm_attr_one<1, EPI, 2>()) != cudaSuccess) return e;
-        if ((e = gemm_attr_one<2, EPI, 2>()) != cudaSuccess) return e;
-        if ((e = gemm_attr_one<4, EPI, 2>()) != cudaSuccess) return e;
-        if ((e = gemm_attr_one<8, EPI, 2>()) != cudaSuccess) return e;
+    if ((e = gemm_attr_nt<EPI, 1, false>()) != cudaSuccess) return e;
+    if constexpr (gemm_epi_tiled(EPI)) {
+        if ((e = gemm_attr_nt<EPI, 2, false>()) != cudaSuccess) return e;
+        if ((e = gemm_attr_nt<EPI, 1, true>()) != cudaSuccess) return e;
+        if ((e = gemm_attr_nt<EPI, 2, true>()) != cudaSuccess) return e;
+        if ((e = gemm_attr_nt<EPI, 3, true>()) != cudaSuccess) return e;
     }
     return cudaSuccess;
 }
 
-// 32-feature tiles for a GEMM?  Only the big ones (their k-loop is bound by activation re-reads), only when the grid
-// still covers ~90 % of the SMs and the 32-row weight slab fits.  ACB_LM_FT32=0 turns it off.
-static int pick_ft2(int N, int K, int nsplit, int kslice, int nt, int sms) {
+// Tiling of one decode GEMM, from its shape and the SM's shared memory:
+//  * big GEMMs (>= 2 M weights; d x d at d = 1536 qualifies) take the narrowest of the 32- and 48-feature staged tilings whose grid
+//    runs in ONE wave and still covers >= 80 % of the SMs.  With the 16-row activation block staged next to the weight slab, a
+//    32-feature CTA of FFN1 / FFN2 needs ~159 KB, one per SM: 192 CTAs would be 1.3 waves, their 128 48-feature CTAs are one.
+//  * other GEMMs (and every GEMM with ACB_LM_FT32=0) take 16-feature staged tiles when those run in one wave;
+//  * otherwise (heads at N = 8192: 256 x 159 KB or no 48-feature split; prefill's 64-row blocks) the activations are loaded
+//    into registers, with 32-feature tiles for big GEMMs when the grid covers ~90 % of the SMs and two CTAs share an SM.
+// Feature tiles never change a sum (same kslice, same per-warp k ranges), so every choice is bit-identical.
+static GemmTiling pick_tiling(const acb_lm* lm, int N, int K, int nsplit, int kslice, int nt) {
     const char* e = getenv("ACB_LM_FT32");
-    const bool enabled = !(e && e[0] == '0');
-    if (!enabled || N % 32 != 0 || (size_t)N * K < ((size_t)2 << 20)) return 1;   // d x d at d = 1536 qualifies (2.36 M weights)
-    if ((N / 32) * nsplit * 10 < sms * 9) return 1;
-    if (gemm_smem_bytes(nt, kslice, 2) > (size_t)GEMM_MAX_SMEM) return 1;
-    return 2;
+    const bool wide = !(e && e[0] == '0') && (size_t)N * K >= ((size_t)2 << 20);
+    auto one_wave = [&](int ft2, bool staged) {
+        const size_t smem = gemm_smem_bytes(nt, kslice, ft2, staged);
+        if (N % (16 * ft2) != 0 || smem > (size_t)GEMM_MAX_SMEM) return false;
+        const int per_sm = (int)((size_t)lm->smem_per_sm / (smem + 1024));   // + the 1 KB the runtime reserves per block
+        return (N / (16 * ft2)) * nsplit <= lm->sms * per_sm;
+    };
+    if (wide) {
+        for (int ft2 = 2; ft2 <= 3; ++ft2)
+            if (one_wave(ft2, true) && (N / (16 * ft2)) * nsplit * 10 >= lm->sms * 8) return {ft2, true};
+    } else if (one_wave(1, true)) {
+        return {1, true};
+    }
+    if (wide && N % 32 == 0 && (N / 32) * nsplit * 10 >= lm->sms * 9 &&
+        gemm_smem_bytes(nt, kslice, 2, false) <= (size_t)GEMM_REG_MAX_SMEM)
+        return {2, false};
+    return {1, false};
 }
 
 // K-slices per GEMM: the slab a CTA stages (16 x kslice fp16) must fit ~64 KB of shared memory, and when the
@@ -1081,10 +1193,15 @@ static int enqueue_step_kernels(acb_lm* lm, cudaStream_t s, float* logits_out, i
     const bool pdl = lm->pdl;
     int nl = 0, ks = 0;
 
+    // The first kernel of a step (or prefill pass) is launched WITHOUT the PDL attribute, so it starts only after everything
+    // enqueued before it has completed: the previous step's sampler (which advances pos), acb_lm_begin's cross K/V GEMMs,
+    // a prefill pass.  Every later kernel of the step starts after it, so within the step pos is constant and so are the cache
+    // positions < pos and the cross K/V -- lm_attn2_kernel and lm_cross_attn_kernel read them before griddepcontrol.wait.
+    // (A graph replay starts with the same full dependency.)
     if (!gemms_only) {
-        if (pf) ACB_LAUNCH(lm_embed_kernel<true>, dim3(rows), dim3(256), 0, s, pdl, (const __half*)lm->w.emb, lm->w.inv_freq,
+        if (pf) ACB_LAUNCH(lm_embed_kernel<true>, dim3(rows), dim3(256), 0, s, false, (const __half*)lm->w.emb, lm->w.inv_freq,
                            (const int64_t*)B.seq, (const int*)B.pos, B.x, d, c.n_q, c.card, c.max_seq, lm->batch, c.pos_scale, rows_real);
-        else ACB_LAUNCH(lm_embed_kernel<false>, dim3(rows), dim3(256), 0, s, pdl, (const __half*)lm->w.emb, lm->w.inv_freq,
+        else ACB_LAUNCH(lm_embed_kernel<false>, dim3(rows), dim3(256), 0, s, false, (const __half*)lm->w.emb, lm->w.inv_freq,
                         (const int64_t*)B.seq, (const int*)B.pos, B.x, d, c.n_q, c.card, c.max_seq, lm->batch, c.pos_scale, rows);
         ++nl;
         DBG("lm_embed_kernel", -1);
@@ -1125,9 +1242,9 @@ static int enqueue_step_kernels(acb_lm* lm, cudaStream_t s, float* logits_out, i
         const int ns = pick_split(N, K, lm->sms, true, &ks);
         GemmParams p = base_gemm(W, X, N, K, rows, ks);
         p.out_f32 = B.part; p.ld_out = N; p.split_stride = part_stride;
-        const int ft2 = pick_ft2(N, K, ns, ks, nt, lm->sms);
-        p.timing = tl(id == G_O ? "gemm_O" : (id == G_CQ ? "gemm_CQ" : (id == G_CO ? "gemm_CO" : "gemm_FFN2")), layer, (N / (16 * ft2)) * ns);
-        ACB_TRY(launch_gemm<EPI_PARTIAL>(nt, p, ns, s, pdl, ft2));
+        const GemmTiling t = pick_tiling(lm, N, K, ns, ks, nt);
+        p.timing = tl(id == G_O ? "gemm_O" : (id == G_CQ ? "gemm_CQ" : (id == G_CO ? "gemm_CO" : "gemm_FFN2")), layer, (N / (16 * t.ft2)) * ns);
+        ACB_TRY(launch_gemm<EPI_PARTIAL>(nt, p, ns, s, pdl, t));
         ++nl;
         DBG("gemm_EPI_PARTIAL", layer);
         pending = ns;
@@ -1142,10 +1259,10 @@ static int enqueue_step_kernels(acb_lm* lm, cudaStream_t s, float* logits_out, i
             GemmParams p = base_gemm((const __half*)lm->w.w_qkv + (size_t)l * 3 * d * d, B.h16, 3 * d, d, rows, ks);
             p.q32 = B.q32; p.kc = (__half*)B.k_cache + l * kv_layer; p.vc = (__half*)B.v_cache + l * kv_layer;
             p.d = d; p.H = H; p.cache_len = c.max_seq; p.pos = B.pos; p.rows_real = rows_real;
-            const int ft2 = pf ? 1 : pick_ft2(3 * d, d, 1, ks, nt, lm->sms);
-            p.timing = tl("gemm_QKV", l, 3 * d / (16 * ft2));
-            if (pf) ACB_TRY(launch_gemm<EPI_QKV_PF>(nt, p, 1, s, pdl, 1));
-            else ACB_TRY(launch_gemm<EPI_QKV>(nt, p, 1, s, pdl, ft2));
+            const GemmTiling t = pf ? GemmTiling{1, false} : pick_tiling(lm, 3 * d, d, 1, ks, nt);
+            p.timing = tl("gemm_QKV", l, 3 * d / (16 * t.ft2));
+            if (pf) ACB_TRY(launch_gemm<EPI_QKV_PF>(nt, p, 1, s, pdl, t));
+            else ACB_TRY(launch_gemm<EPI_QKV>(nt, p, 1, s, pdl, t));
             ++nl;
             DBG("gemm_EPI_QKV", l);
         }
@@ -1191,9 +1308,9 @@ static int enqueue_step_kernels(acb_lm* lm, cudaStream_t s, float* logits_out, i
             pick_split(ffn, d, lm->sms, false, &ks);
             GemmParams p = base_gemm((const __half*)lm->w.w_ff1 + (size_t)l * ffn * d, B.h16, ffn, d, rows, ks);
             p.out_f16 = (__half*)B.f16; p.ld_out = ffn;
-            const int ft2 = pick_ft2(ffn, d, 1, ks, nt, lm->sms);
-            p.timing = tl("gemm_FFN1", l, ffn / (16 * ft2));
-            ACB_TRY(launch_gemm<EPI_GELU>(nt, p, 1, s, pdl, ft2)); ++nl;
+            const GemmTiling t = pick_tiling(lm, ffn, d, 1, ks, nt);
+            p.timing = tl("gemm_FFN1", l, ffn / (16 * t.ft2));
+            ACB_TRY(launch_gemm<EPI_GELU>(nt, p, 1, s, pdl, t)); ++nl;
             DBG("gemm_EPI_GELU", l);
         }
         ACB_TRY(partial_gemm((const __half*)lm->w.w_ff2 + (size_t)l * d * ffn, B.f16, d, ffn, l, G_FF2));
@@ -1208,7 +1325,7 @@ static int enqueue_step_kernels(acb_lm* lm, cudaStream_t s, float* logits_out, i
         pick_split(N, d, lm->sms, false, &ks);
         GemmParams p = base_gemm(lm->w.heads, B.h16, N, d, rows, ks);
         p.out_f32 = B.logits; p.ld_out = N;
-        ACB_TRY(launch_gemm<EPI_F32>(nt, p, 1, s, pdl, pick_ft2(N, d, 1, ks, nt, lm->sms))); ++nl;
+        ACB_TRY(launch_gemm<EPI_F32>(nt, p, 1, s, pdl, pick_tiling(lm, N, d, 1, ks, nt))); ++nl;
         DBG("gemm_EPI_F32", -1);
     }
     if (!gemms_only) {
@@ -1271,9 +1388,10 @@ extern "C" int acb_lm_create(const acb_lm_config* cfg, const acb_lm_weights* w, 
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&lm->sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaDeviceGetAttribute(&lm->smem_per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev);
     cudaError_t e = cudaStreamCreateWithFlags(&lm->capture_stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) { delete lm; acb_set_error("acb_lm_create: cudaStreamCreate: %s", cudaGetErrorString(e)); return ACB_ERR_CUDA; }
-    // the GEMMs stage up to ~70 KB of weights per CTA; keep the shared-memory carve-out at its maximum for every kernel
+    // the GEMMs stage up to ~210 KB of weights and activations per CTA; keep the shared-memory carve-out at its maximum for every kernel
     // of the step so that co-resident kernels (PDL) never force an L1/shared reconfiguration.
     cudaError_t ea = gemm_attr_all<EPI_PARTIAL>();
     if (ea == cudaSuccess) ea = gemm_attr_all<EPI_QKV>();
